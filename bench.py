@@ -18,6 +18,8 @@ per-view loss scalars at the end of the timed region.
   python bench.py --impl reference --gpus N ...            # the UNMODIFIED reference CUDA extension
                                                            # (oracle/_ref/_refC.so) driven by the same loop;
                                                            # loads nothing of this framework's native code
+  python bench.py ... --dump-outputs DIR                   # also write what the last timed step computed as
+                                                           # DIR/<name>.npy, to compare two builds output for output
 
 Prints ONE JSON line on rank 0 (see DESIGN.md, Measurement, for every key).
 """
@@ -64,7 +66,50 @@ def parse():
     ap.add_argument("--train", type=int, default=0, help="data-parallel training step instead of independent views")
     ap.add_argument("--views-per-step", type=int, default=2, help="--train: views per rank per optimizer step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (the render's result dict, "
+                         "depth->normal map, loss, parameter gradients; --train: the updated parameters) as "
+                         f"DIR/<name>.npy in float32 / float64; an array of more than {DUMP_MAX_ELEMENTS} elements as "
+                         "that many of them at fixed seeded positions")
     return ap.parse_args()
+
+
+DUMP_MAX_ELEMENTS = 1 << 19
+DUMP_MAX_BYTES = 64 << 20
+PARAM_NAMES = ("xyz", "scale", "rot", "opacity", "f_dc", "f_rest")
+
+
+def collect_outputs(out, normal, loss, grads):
+    """Name -> tensor of what a caller of one step receives: the render's result dict (+ the screen-space gradient),
+    the depth->normal map, the loss and the gradients of the Gaussian parameters (those that have one)."""
+    res = {k: v for k, v in out.items() if torch.is_tensor(v)}
+    vs = out.get("viewspace_points")
+    if torch.is_tensor(vs) and vs.grad is not None:
+        res["viewspace_points_grad"] = vs.grad
+    res["normal"], res["loss"] = normal, loss
+    for name, g in zip(PARAM_NAMES, grads):
+        if g is not None:
+            res["grad_" + name] = g
+    return res
+
+
+def dump_outputs(directory, tensors):
+    """Write each tensor as <directory>/<name>.npy (float64 stays float64, everything else becomes float32); a tensor of
+    more than DUMP_MAX_ELEMENTS elements is written as that many of its flattened elements at sorted positions drawn
+    with a fixed seed, so that two runs with the same arguments write comparable files."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    total = 0
+    for name, t in tensors.items():
+        t = t.detach().reshape(-1)
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMENTS, replace=False))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32)
+        total += a.nbytes
+        if total > DUMP_MAX_BYTES:
+            raise RuntimeError(f"--dump-outputs: more than {DUMP_MAX_BYTES} bytes")
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -284,6 +329,7 @@ def run_reference(a):
     loss_fn = make_loss(dev, H, W)
     params = model.parameters_list()
     bg = torch.zeros(3, device=dev)  # the reference dereferences bg on the device in backward (backward.cu:586)
+    last = {}
 
     def render(cam):
         xyz, shs, opacity, scales, rotations = ref_torch_ops.gaussian_properties(model)
@@ -293,13 +339,16 @@ def run_reference(a):
                                     False, False)
         color, radii, depth, median, opac = ref_driver.rasterize(rs, xyz, m2d, opacity, shs=shs, scales=scales,
                                                                  rotations=rotations)
-        return {"render": color, "rendered_depth": depth, "rendered_final_opacity": opac, "radii": radii}
+        return {"render": color, "rendered_depth": depth, "rendered_final_opacity": opac, "radii": radii,
+                "viewspace_points": m2d}
 
     def step(cam):
         if not backward:
             with torch.no_grad():
                 out = render(cam)
                 n = ref_torch_ops.depth2normal(out["rendered_depth"][0], cam.K)
+            if a.dump_outputs:
+                last.update(out=out, normal=n)
             return out["rendered_depth"].mean() + 0.0 * n[0, 0, 0]
         for p in params:
             p.grad = None
@@ -307,6 +356,8 @@ def run_reference(a):
         loss = loss_fn(out)
         loss.backward()
         n = ref_torch_ops.depth2normal(out["rendered_depth"].detach()[0], cam.K)
+        if a.dump_outputs:
+            last.update(out=out, normal=n)
         return loss.detach() + 0.0 * n[0, 0, 0]
 
     for i in range(max(Wn, 3)):
@@ -329,6 +380,8 @@ def run_reference(a):
     torch.cuda.synchronize(dev)
     ms_dev = e0.elapsed_time(e1)
     clocks = sampler.stop()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, collect_outputs(last["out"], last["normal"], losses[K - 1], [p.grad for p in params]))
 
     host_loss = torch.zeros(K).pin_memory()
     e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -389,6 +442,7 @@ def run_new(a):
     params = model.parameters_list()
     renderer = renderers.make({"name": "vanilla_renderer", "fused_activations": bool(a.fused)})
     _C.set_pipelined(bool(a.pipelined))
+    last = {}
 
     def normal(cam, depth):
         return ops.depth2normal(depth, cam.fx, cam.fy, cam.cx, cam.cy)
@@ -398,6 +452,8 @@ def run_new(a):
             with torch.no_grad():
                 out = rend.render(cam, model)
                 n = normal(cam, out["rendered_depth"][0])
+            if a.dump_outputs:
+                last.update(out=out, normal=n)
             return out["rendered_depth"].mean() + 0.0 * n[0, 0, 0]
         for p in params:
             p.grad = None
@@ -405,6 +461,8 @@ def run_new(a):
         loss = loss_fn(out)
         loss.backward()
         n = normal(cam, out["rendered_depth"].detach()[0])
+        if a.dump_outputs:
+            last.update(out=out, normal=n)
         return loss.detach() + 0.0 * n[0, 0, 0]
 
     def sync_all():
@@ -494,6 +552,13 @@ def run_new(a):
     clocks = sampler.stop()
     assert bool(torch.isfinite(all_losses).all())
     _C.check_pipeline(wait=True)
+    if a.dump_outputs and rank == 0:
+        grads = [p.grad for p in params]
+        if graphed is not None:  # the static outputs and gradients of the graph that replayed the last step
+            gs = graphed[(K - 1) % nstreams]
+            last.update(out=gs.out if backward else gs.loss, normal=gs.extra)
+            grads = gs.grads if backward else []
+        dump_outputs(a.dump_outputs, collect_outputs(last["out"], last["normal"], losses[K - 1], grads))
 
     # ---------------- leg 1b: per-kernel CUDA-event times over the same K steps (library-side events around every
     # launch on the caller's stream; eager launches, one stream).  Kept out of leg 1. ----------------
@@ -839,6 +904,8 @@ def run_train(a, _C, L, parallel, model, hcams, c, nviews_total, step, renderer,
         sync_all()
         return parallel.barrier_max_ms(e0.elapsed_time(e1), dev) / K
     res["with_comm"] = timed(True)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, {"param_" + n: p for n, p in zip(PARAM_NAMES, params)})
     ident = None
     if world > 1:
         chk = torch.stack([p.detach().double().sum() for p in params] + [p.detach().double().abs().sum() for p in params])

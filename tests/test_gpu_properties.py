@@ -1,8 +1,11 @@
 """Size-independent properties at BASELINE.json's full size (cfg 3: 1M Gaussians, 1920x1080)."""
 import math
 
+import numpy as np
 import pytest
 import torch
+
+import gpu_util as U
 
 pytestmark = pytest.mark.gpu
 
@@ -109,21 +112,19 @@ def test_backward_linearity_full_size(big):
 
 
 def test_full_size_forward_bit_exact_vs_reference(big):
-    """cfg 3 at full size (1M Gaussians, 1080p): all five forward outputs and num_rendered are bit-identical to the
-    unmodified reference extension on the same device; gradients of a random cotangent within 1e-3."""
-    from oracle import ref_driver
-    if not ref_driver.available():
-        pytest.skip("oracle/_ref/_refC.so not present")
+    """cfg 3 at full size (1M Gaussians, 1080p): all five forward outputs and num_rendered are bit-identical to what the
+    unmodified reference extension computed on a B200; gradients of a random cotangent within 1e-3 (on the stored
+    seeded sample of the reference's, tests/golden/ref_outputs_sampled.npz)."""
     from gaustudio_b200 import _C
     from gaustudio_b200.rasterizer import GaussianRasterizationSettings, GaussianRasterizer
     model, cams, c, dev = big
     cam = cams[0]
     a = _args(model, cam, c, dev)
+    G = np.load(U.SAMPLED)
     new = _C.rasterize_gaussians(*a)
-    ref = ref_driver.module().rasterize_gaussians(*a)
-    assert new[0] == ref[0]
+    assert new[0] == int(G["cfg3full_R"])
     for i, name in zip(range(1, 6), ("color", "depth", "median", "opacity", "radii")):
-        assert torch.equal(new[i], ref[i]), name
+        assert U.digest(new[i]) == G["cfg3full_" + name], name
     rs = GaussianRasterizationSettings(c["H"], c["W"], math.tan(cam.FoVx * 0.5), math.tan(cam.FoVy * 0.5),
                                        torch.zeros(3, device=dev), 1.0, cam.world_view_transform,
                                        cam.full_proj_transform, 3, cam.camera_center, False, False)
@@ -139,8 +140,7 @@ def test_full_size_forward_bit_exact_vs_reference(big):
         ((color * wc).sum() + (depth * wd).sum() + opac.sum()).backward()
         return [t.grad for t in (xyz, op, sc, rot, sh)]
     gn = grads(lambda rs_, *a_, **k: GaussianRasterizer(rs_)(*a_, **k))
-    gr = grads(ref_driver.rasterize)
-    for name, x, y in zip(("xyz", "opacity", "scale", "rot", "sh"), gn, gr):
-        scale = float(y.abs().max())
-        bad = ((x - y).abs() > 1e-3 * y.abs() + 1e-4 * scale).float().mean()
+    for name, x in zip(("xyz", "opacity", "scale", "rot", "sh"), gn):
+        x, y, scale = U.load_sample(G, "cfg3full_g_" + name, x)
+        bad = (np.abs(x - y) > 1e-3 * np.abs(y) + 1e-4 * scale).mean()
         assert float(bad) < 1e-5, (name, float(bad))
